@@ -3,7 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W [--impl reference] [--precision fp16|fp32]
                     [--config mnist|fmnist|celeba] [--batch B --rec_rr R --rec_iters L]
-                    [--scaling weak|strong] [--no_extra] [--no_profile]
+                    [--scaling weak|strong] [--no_extra] [--no_profile] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one batch of synthetic images: one `gan.reconstruct` call =
 R restarts x L momentum-GD steps of generator forward + MSE + backward-to-z, then arg-min select.
@@ -24,6 +24,12 @@ D2H of the reconstructions inside the timed region); `roofline` = the dominant k
 events around each launch on the launching stream, in a separate pass) against the measured bf16 tensor peak in
 MEASURED_PEAKS.json; `cpu_baseline` = the oracle restatement of the reference's TF1 CPU path on this box's host
 cores (bounded sample).  `--impl reference` times only that CPU port (the reference itself cannot run: no TF1/py2).
+
+The inputs are drawn on the host from fixed seeds (the generator's forward in float64 by the CPU oracle), so the same
+arguments give the same inputs on every run and with every build of the library.  `--dump-outputs DIR` writes what the
+last timed step returned to its caller, the reconstructions, as DIR/reconstructions.npy (float32): two builds can then
+be compared output for output.  An output over 64 MiB is replaced by a fixed, seeded sample of its images, whose indices
+go to DIR/reconstructions_rows.npy.
 """
 import argparse
 import json
@@ -51,6 +57,8 @@ C5_GLOBAL_BATCH = 4096                    # configs[4]: MNIST R=10 L=200, batch 
 C5_PER_GPU = C5_GLOBAL_BATCH // 8
 FMNIST_WEIGHT_SEED = 11241991             # synthetic C3 differs from C2 only in the weights (SURVEY 8d)
 FALLBACK_PEAKS = {"bf16_tflops": 1590.0, "bf16_tflops_sustained": 1400.0, "hbm_gbs": 6650.0}
+DUMP_BYTES = 64 * 2 ** 20 - 4096          # --dump-outputs: all files together, .npy headers included, stay under 64 MiB
+DUMP_SAMPLE_SEED = 0
 
 
 def load_peaks():
@@ -63,6 +71,22 @@ def load_peaks():
     d = dict(FALLBACK_PEAKS)
     d["_source"] = "fallback"
     return d
+
+
+def dump_output(out_dir, name, t):
+    """Write `t` as out_dir/<name>.npy in float32.  Above DUMP_BYTES only a fixed, seeded sample of its leading-axis rows
+    is written (the same rows for the same shape), and out_dir/<name>_rows.npy holds their indices (float64)."""
+    a = t.detach().float().cpu().numpy()
+    os.makedirs(out_dir, exist_ok=True)
+    if a.nbytes > DUMP_BYTES:
+        row_bytes = a.nbytes // a.shape[0]
+        n = DUMP_BYTES // (row_bytes + 8)
+        rows = np.sort(np.random.default_rng(DUMP_SAMPLE_SEED).choice(a.shape[0], n, replace=False))
+        np.save(os.path.join(out_dir, name + "_rows.npy"), rows.astype(np.float64))
+        a = a[rows]
+    path = os.path.join(out_dir, name + ".npy")
+    np.save(path, a)
+    return path
 
 
 class ClockSampler:
@@ -310,14 +334,17 @@ class Workload:
         self.gan.rec_rr, self.gan.rec_iters, self.gan.rec_lr = R, L, 10.0
         self.hwc = int(np.prod(self.gan.image_dim))
         self.B_global = B_local * world
-        # synthetic inputs (SURVEY 8d, S1: on-manifold + noise): generated ON DEVICE by the native generator
+        # synthetic inputs (SURVEY 8d, S1: on-manifold + noise): G(z*) by the float64 CPU oracle, not by the library under
+        # test, so that every build is fed the same images
+        from oracle import defensegan_oracle as O
         g = torch.Generator(device="cpu").manual_seed(1990)
         sig = (1.0 / self.gan.latent_dim) ** 0.5
         zstar = torch.randn(self.B_global, self.gan.latent_dim, generator=g) * sig
         eps = torch.randn(self.B_global, *self.gan.image_dim, generator=g)
         lo = -1.0 if dataset == "celeba" else 0.0
-        chunks = [self.gan.generator_fn(zstar[i:i + 512].to(dev)) for i in range(0, self.B_global, 512)]
-        self.x_full = (torch.cat(chunks) + 0.1 * eps.to(dev)).clamp_(lo, 1.0).contiguous()
+        with torch.no_grad():
+            on_manifold = O.generator_forward(dataset, O.weights_to_torch(self.gan.weights, torch.float64), zstar.double())
+        self.x_full = (on_manifold.float() + 0.1 * eps).clamp_(lo, 1.0).to(dev).contiguous()
         self.z0_full = (torch.randn(self.B_global * R, self.gan.latent_dim, generator=g) * sig).to(dev)
         self.x_host = self.x_full.cpu().pin_memory()
         self.out_host = torch.empty_like(self.x_host).pin_memory()
@@ -345,7 +372,8 @@ class Workload:
 
 
 def timed(fn, steps, warmup, dev, flush, distributed):
-    """ms for `steps` calls of fn, CUDA events, barrier + synchronize on both sides, max over ranks."""
+    """(ms for `steps` calls of fn, CUDA events, barrier + synchronize on both sides, max over ranks; what the last call
+    returned)."""
     import torch.distributed as dist
 
     def barrier():
@@ -360,15 +388,18 @@ def timed(fn, steps, warmup, dev, flush, distributed):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     barrier()
     e0.record()
-    for _ in range(steps):
+    for i in range(steps):
         flush.zero_()                      # > L2 capacity written between timed iterations (inside the bracket)
-        fn()
+        if i + 1 < steps:
+            fn()                           # dropped at once, so the next step can reuse its memory
+        else:
+            last = fn()
     e1.record()
     barrier()
     t = torch.tensor([e0.elapsed_time(e1)], dtype=torch.float64, device=dev)
     if distributed:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
-    return float(t.item())
+    return float(t.item()), last
 
 
 def kernel_breakdown(wl, peaks, precision):
@@ -462,7 +493,12 @@ def _main(out):
     ap.add_argument("--cpu_sample", type=int, default=64, help="images of the cpu_baseline sample (0 = skip)")
     ap.add_argument("--no_profile", action="store_true")
     ap.add_argument("--no_extra", action="store_true", help="skip the configs[2]/[3]/[4]-share and batch-50 sub-measurements")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's reconstructions to DIR (GPU arm)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what the GPU arm computed; the reference arm has no such output")
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -472,7 +508,7 @@ def _main(out):
         return
     if world != args.gpus and world > 1:
         raise SystemExit("--gpus %d does not match WORLD_SIZE %d" % (args.gpus, world))
-    if args.steps < 1 or args.warmup < 3:
+    if args.warmup < 3:
         print("note: the timing rules ask for >= 3 warm-up steps", file=sys.stderr)
 
     import torch.distributed as dist
@@ -497,14 +533,17 @@ def _main(out):
     torch.cuda.synchronize(dev)
     if rank == 0:
         sampler.start()
-    ms = timed(wl.step, args.steps, 0, dev, flush, distributed)
+    ms, last_rec = timed(wl.step, args.steps, 0, dev, flush, distributed)
     clocks = sampler.stop() if rank == 0 else None
     launches_per_step = wl.gan._native.last_launch_count
     enqueues_per_call = wl.gan._native.last_enqueue_count
     value = wl.B_global * args.steps / (ms / 1000.0)
+    if args.dump_outputs and rank == 0:
+        print("wrote", dump_output(args.dump_outputs, "reconstructions", last_rec), file=sys.stderr)
+    del last_rec
 
     # ---- end-to-end through the public API with HOST buffers (`e2e`) ------------------------------------
-    ms_e2e = timed(wl.e2e_step, args.steps, max(1, min(args.warmup, 2)), dev, flush, distributed)
+    ms_e2e, _ = timed(wl.e2e_step, args.steps, max(1, min(args.warmup, 2)), dev, flush, distributed)
     e2e_value = wl.B_global * args.steps / (ms_e2e / 1000.0)
 
     peaks = load_peaks()
@@ -522,8 +561,8 @@ def _main(out):
 
         def sub(ds, b, seed=None):
             w2 = Workload(ds, b, R, L, args.precision, dev, 0, 1, weight_seed=seed)
-            m = timed(w2.step, k, 3, dev, flush, False)
-            me = timed(w2.e2e_step, k, 1, dev, flush, False)
+            m, _ = timed(w2.step, k, 3, dev, flush, False)
+            me, _ = timed(w2.e2e_step, k, 1, dev, flush, False)
             macs = w2.gan._native.macs_per_row
             r = {"workload": workload_name(ds, b, R, L), "value": b * k / (m / 1e3), "ms_per_step": m / k, "steps": k,
                  "e2e": b * k / (me / 1e3), "gpu_launches_per_step": w2.gan._native.last_launch_count,
